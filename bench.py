@@ -27,6 +27,8 @@ Weights are random-init at the real 1.7B geometry, inputs synthetic (no checkpoi
   cpu_baseline / --impl reference: the CPU oracle (torch eager fp32, dynamic KV) on a bounded sample, host threads
   --sweep      chunk (BASELINE config 5: chunk_size in {1,2,4,8,16}) / prompt (TTFA over P in {10,40,96,232} split
                into prefill, first chunk, first window) ; --size 0.6B = config 2
+  --dump-outputs DIR  what the last timed step returned: its PCM (pcm.npy, float32, with the chunk lengths in
+               chunk_samples.npy), or its codes with --no-codec (codes.npy); seeded inputs, so two builds can be compared
 """
 from __future__ import annotations
 
@@ -73,7 +75,30 @@ def parse():
     ap.add_argument("--sweep", default="none", choices=["none", "chunk", "prompt", "all"])
     ap.add_argument("--num-ctas", type=int, default=0)
     ap.add_argument("--cpu-frames", type=int, default=64)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (PCM, or codes with --no-codec) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    return args
+
+
+DUMP_BUDGET = 64 << 20   # bytes, all dumped arrays together
+
+
+def dump_outputs(out_dir, arrays):
+    """Save each array as out_dir/<name>.npy.  Above DUMP_BUDGET in all, each array is replaced by the same fixed, seeded
+    sample of its flattened elements (in order), so that two runs with the same arguments stay comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BUDGET:
+            keep = a.size * DUMP_BUDGET // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -272,8 +297,9 @@ def run_b200(args):
     kw = dict(max_new_tokens=args.frames, min_new_tokens=args.frames, chunk_size=args.chunk)
     chunk_ms, ttfa_ms = [], []
 
-    def step_resident(timed: bool, chunk=None, prompt=None):
-        """prompt resident in HBM; codes -> PCM per chunk on device.  Returns frames."""
+    def step_resident(timed: bool, chunk=None, prompt=None, keep=None):
+        """prompt resident in HBM; codes -> PCM per chunk on device.  Returns frames.  `keep`: a list that receives a
+        device copy of every chunk the caller gets (PCM, or codes without the codec)."""
         torch.manual_seed(rank * 1000 + len(ttfa_ms))
         e0 = torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -289,6 +315,8 @@ def run_b200(args):
                 first = torch.cuda.Event(enable_timing=True)
                 first.record()
             n += t["chunk_steps"]
+            if keep is not None:
+                keep.append(pcm.clone())
             if timed and "kernel_ms" in t:
                 chunk_ms.append(t["kernel_ms"])
         if timed and first is not None:
@@ -329,13 +357,20 @@ def run_b200(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     frames = 0
-    for _ in range(args.steps):
-        frames += step_resident(True)
+    last = [] if args.dump_outputs and rank == 0 else None
+    for i in range(args.steps):
+        frames += step_resident(True, keep=last if i == args.steps - 1 else None)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count + model.codec_launches() - l0
     clk = clocks.stop() if rank == 0 else None
+    if last is not None:
+        if args.no_codec:   # codes [frames, 16] per chunk
+            dump_outputs(args.dump_outputs, {"codes": torch.cat(last).cpu().double().numpy()})
+        else:               # 24 kHz PCM per chunk: the samples in order, and where the chunks split them
+            dump_outputs(args.dump_outputs, {"pcm": torch.cat(last).float().cpu().numpy(),
+                                             "chunk_samples": np.array([c.numel() for c in last], dtype=np.float64)})
     # ---- extra leg: the same request with the STATEFUL streaming codec (SURVEY 8(f) item 2; not the headline: its
     # Phase-2 audio is the non-streaming decode rather than the reference's 25-frame-context windows)
     sc = None

@@ -31,16 +31,18 @@ class _FakeReq:
 
 
 class _FakeSched:
-    """max_batch slots; every step emits min(n, remaining) 'frames' whose values identify (request, frame)."""
+    """max_batch slots; every step emits min(n, remaining) 'frames' whose values identify (request, frame).  Admits
+    nothing until `admitting` is set."""
 
     def __init__(self, max_batch):
         self.max_batch, self.active, self.peak, self.batch_sizes = max_batch, {}, 0, []
+        self.admitting = threading.Event()
 
     def __len__(self):
         return len(self.active)
 
     def has_capacity(self):
-        return len(self.active) < self.max_batch
+        return self.admitting.is_set() and len(self.active) < self.max_batch
 
     def submit(self, tie, tam, tth, tpe, tag=None, max_new_tokens=0, **kw):
         if tie is None:
@@ -86,6 +88,11 @@ def test_continuous_batcher_join_leave_and_isolation():
         th = threading.Thread(target=client, args=(i, n))
         th.start()
         threads.append(th)
+        if i == 2:   # the first three requests are admitted together, so all slots are busy at once whatever the timing
+            deadline = time.time() + 10
+            while b.pending.qsize() < 3 and time.time() < deadline:
+                time.sleep(0.0005)
+            sched.admitting.set()
         time.sleep(0.002 * (i % 3))   # staggered arrivals: some join while others are mid-stream
     bad = b.submit(lambda: (None, 0, 0, 0, None), max_new_tokens=5)
     with pytest.raises(ValueError):
